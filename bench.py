@@ -2,7 +2,7 @@
 """bench.py -- the headline benchmark: point-clouds/sec, SampleNet forward (train mode: generator -> soft projection)
 + Chamfer simplification loss at B=32 per GPU, N=1024 -> 64, k=8 (BASELINE.json metric; registration flavour).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P bench.py --gpus N ...
 
 Prints ONE JSON line from rank 0 (see the repo task contract).  Key points:
@@ -15,7 +15,9 @@ Prints ONE JSON line from rank 0 (see the repo task contract).  Key points:
     timing = max over ranks of CUDA-event time;
   * `roofline`: the dominant kernel timed live with CUDA events; `cpu_baseline`: the same step on the host cores
     (torch CPU layer stack + C oracle kNN/projection + the reference's own CPU Chamfer from oracle/_ref);
-  * `--impl reference`: that CPU path as the measured arm (all host threads).
+  * `--impl reference`: that CPU path as the measured arm (all host threads);
+  * `--dump-outputs DIR`: after the timed steps, rank 0 writes what the last step of the `value` leg returned (simp, proj, loss) as
+    DIR/<name>.npy in float32.  Inputs and weights are seeded, so two builds run with the same arguments can be compared output for output.
 """
 import argparse
 import json
@@ -333,7 +335,14 @@ def run_ours(args, rank, world, local_rank):
         vpipe.run_async(dev_pool[i % pool_n])
     ms_single = timed_region(lambda i: step(dev_pool[(args.warmup + i) % pool_n]), args.steps)
     sampler = ClockSampler(local_rank) if rank == 0 else None
-    ms_val = timed_region(lambda i: vpipe.run_async(dev_pool[(args.warmup + i) % pool_n]), args.steps)
+    last = {}
+
+    def value_step(i):
+        last["slot"] = vpipe.run_async(dev_pool[(args.warmup + i) % pool_n])
+
+    ms_val = timed_region(value_step, args.steps)
+    if args.dump_outputs and rank == 0:   # the slot's static buffers are rewritten only by its own replays, none of which follow
+        outputs = {name: getattr(last["slot"], name).detach().float().cpu().numpy() for name in ("simp", "proj", "loss")}
     # ---- e2e leg: pinned host batch -> device, step, loss -> host, every step, through the public streaming API
     #      (PipelinedHostStep: two steps in flight, H2D on a copy stream; every step's loss is read on the host).  The timed region
     #      starts and ends with an EMPTY pipeline: exactly K steps are submitted, launched and finished inside it.
@@ -462,6 +471,10 @@ def run_ours(args, rank, world, local_rank):
         "gpu_reference": gpu_ref,
     }
     print(json.dumps(line), flush=True)
+    if args.dump_outputs:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, a in outputs.items():
+            np.save(os.path.join(args.dump_outputs, name + ".npy"), a)
 
 
 def main():
@@ -470,6 +483,8 @@ def main():
     ap.add_argument("--steps", type=int, default=200)
     ap.add_argument("--warmup", type=int, default=20)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the outputs of the last timed step (value leg, rank 0) to DIR/<name>.npy")
     args = ap.parse_args()
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))

@@ -1,7 +1,8 @@
 """GPU parity tests (run on the B200 box with `-m gpu`): the CUDA path, called through the C-ABI library via the
 package's public API, against the CPU oracle on the same seeded inputs, against the committed golden fixtures
 (generated from the reference's own Python classes, tests/golden/make_golden.py), against the reference's own CPU code
-compiled into oracle/_ref, and -- at BASELINE.json's full sizes -- through size-independent properties.
+compiled into oracle/_ref (its results on these inputs stored in tests/golden/reference_cpu.npz by tests/golden/make_ref_golden.py),
+and -- at BASELINE.json's full sizes -- through size-independent properties.
 
 Bars: indices bit-exact; squared distances bit-exact against the oracle evaluated in the same arithmetic mode
 (SNB200_DIST_FMA <-> oracle contract=True, SNB200_DIST_UNFUSED <-> oracle contract=False == the reference CPU code);
@@ -13,9 +14,9 @@ import numpy as np
 import pytest
 import torch
 
-pytestmark = pytest.mark.gpu
+from oracle import golden
 
-HAVE_REF = os.path.exists(os.path.join(os.path.dirname(__file__), "..", "oracle", "_ref", "libsamplenet_ref.so"))
+pytestmark = pytest.mark.gpu
 
 
 def _t(a, dtype=torch.float32):
@@ -38,9 +39,14 @@ def sb():
     return samplenet_b200
 
 
+@pytest.fixture(scope="module")
+def ref_cpu(golden_dir):
+    return np.load(os.path.join(golden_dir, "reference_cpu.npz"))
+
+
 # ------------------------------------------------------------------------------------------------ Chamfer forward
 @pytest.mark.parametrize("b,n,m", [(1, 1, 1), (2, 64, 1024), (3, 37, 129), (2, 513, 511), (1, 1024, 64), (4, 5, 3), (2, 33, 4099), (1, 6000, 70)])
-def test_chamfer_forward_bitexact(sb, oracle, b, n, m):
+def test_chamfer_forward_bitexact(sb, oracle, ref_cpu, b, n, m):
     r = _rng(b * 1000 + n + m)
     a = r.standard_normal((b, n, 3)).astype(np.float32)
     c = r.standard_normal((b, m, 3)).astype(np.float32)
@@ -53,11 +59,11 @@ def test_chamfer_forward_bitexact(sb, oracle, b, n, m):
         e1, j1, e2, j2 = oracle.nn_distance(a, c, contract=not unfused)
         assert np.array_equal(_n(i1), j1) and np.array_equal(_n(i2), j2)
         assert np.array_equal(_n(d1), e1) and np.array_equal(_n(d2), e2)
-    if HAVE_REF:  # the reference's own CPU code, compiled unmodified
-        d1, i1, d2, i2 = sb.ops.nn_distance_forward(_t(a), _t(c), unfused=True)
-        rd1, ri1, rd2, ri2 = oracle.ref_chamfer_forward(a, c)
-        assert np.array_equal(_n(i1), ri1) and np.array_equal(_n(i2), ri2)
-        assert np.array_equal(_n(d1), rd1) and np.array_equal(_n(d2), rd2)
+    # the reference's own CPU code, compiled unmodified
+    d1, i1, d2, i2 = sb.ops.nn_distance_forward(_t(a), _t(c), unfused=True)
+    key = "chamfer_%d_%d_%d" % (b, n, m)
+    assert golden.digest(i1, i2) == ref_cpu[key + "_idx"]
+    assert golden.digest(d1, d2) == ref_cpu[key + "_dist"]
 
 
 def test_chamfer_lattice_ties(sb, oracle):
@@ -569,7 +575,7 @@ def test_simplification_loss_fused_and_tf_names(sb, oracle):
 
 
 @pytest.mark.parametrize("n,m", [(64, 64), (96, 32), (40, 120), (77, 77), (300, 300), (1024, 1024)])
-def test_emd_exact_mode_bitexact_vs_oracle(sb, oracle, n, m):
+def test_emd_exact_mode_bitexact_vs_oracle(sb, oracle, ref_cpu, n, m):
     """north_star: match ASSIGNMENTS bit-exact.  approx_match(exact=True) (C flag SNB200_EMD_EXACT; env SNB200_EMD_EXACT_EXP=1) evaluates
     the reference's level schedule with the oracle's arithmetic operation for operation (correctly rounded exp, index-order float sums, no
     FMA contraction): the whole `match` tensor -- hence every arg-max assignment -- equals the oracle's bit for bit, and the assignments
@@ -583,9 +589,8 @@ def test_emd_exact_mode_bitexact_vs_oracle(sb, oracle, n, m):
     assert mt.shape == omt.shape == (b, m, n)
     assert np.array_equal(mt.argmax(axis=2), omt.argmax(axis=2)) and np.array_equal(mt.argmax(axis=1), omt.argmax(axis=1))
     assert np.array_equal(mt, omt), np.abs(mt - omt).max()
-    if HAVE_REF and n <= 300:
-        rmt = oracle.ref_approxmatch_cpu(a, c).transpose(0, 2, 1)      # (b, n, m) -> (b, m, n)
-        assert np.array_equal(mt.argmax(axis=2), rmt.argmax(axis=2))
+    if n <= 300:
+        assert np.array_equal(mt.argmax(axis=2), ref_cpu["emd_exact_%d_%d_argmax" % (n, m)])
     # the fast kernel against the exact one: same assignments wherever the exact top-2 gap exceeds the fast kernel's value tolerance
     fast = _n(sb.tf_ops.approx_match(_t(a), _t(c)))
     tol = 2e-3 if n <= 300 else 1e-2      # (the reference's own GPU-vs-CPU self-check flags > 1e-2, approxmatch.cpp:222; the error grows with n)
