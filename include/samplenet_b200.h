@@ -164,13 +164,13 @@ int snb200_encoder_forward(int b, int n, int layout, const float *x, int num_lay
  * 256 points per SM).  Other shapes: one tensor-core launch per layer + a thread-block-cluster FC head.  flags &
  * SNB200_GEN_EXACT_FP32 selects the exact-fp32 CUDA-core conv stack instead (also taken automatically for widths the tensor
  * path does not cover).  b <= 256.  Training-mode pre-BatchNorm activations must stay below ~3e4 in magnitude on the default
- * path (fixed-point statistics exchange); beyond that the call returns NaN rows. */
+ * path (fixed-point statistics exchange); beyond that the call returns NaN rows.  A flag bit not defined below is rejected with
+ * SNB200_EINVAL (64, once a kernel selector, is retired and stays unused). */
 #define SNB200_GEN_EXACT_FP32 1
 #define SNB200_GEN_PER_LAYER_KERNELS 8 /* tensor-core path as one launch per layer instead of the persistent conv-stack kernel */
 #define SNB200_GEN_SEPARATE_HEAD 16 /* keep the pool + FC head as its own thread-block-cluster launch */
 #define SNB200_GEN_WORKSPACE_PRIMED 32 /* the caller keeps `workspace` across calls and its first 256 bytes are zero (freshly zeroed or as the
                                          previous PRIMED call left them): the persistent kernel cleans the rest itself, no memset in front */
-#define SNB200_GEN_CONV_STACK_V1 64 /* the round-1 persistent kernel (128-point tiles, activations as the A operand) instead of the transposed-GEMM one */
 #define SNB200_GEN_PROFILE_SKIP_HEAD 2 /* profiling only: stop after the conv stack (out is not written) */
 #define SNB200_GEN_PROFILE_SKIP_CONV 4 /* profiling only: run only the pool + FC head on whatever the workspace holds */
 size_t snb200_generator_workspace_bytes(int b, int n, int num_conv, const snb200_layer *conv, int num_fc, const snb200_layer *fc);

@@ -88,6 +88,11 @@ static int check_layers(const char *who, int num_layers, const snb200_layer *lay
     return SNB200_OK;
 }
 
+// every SNB200_GEN_* bit the header defines; any other bit is rejected rather than ignored (64 selected a kernel that no longer exists
+// and is not reused, so a caller that still sets it gets an error instead of a different kernel)
+constexpr int kGenFlagsDefined = SNB200_GEN_EXACT_FP32 | SNB200_GEN_PROFILE_SKIP_HEAD | SNB200_GEN_PROFILE_SKIP_CONV | SNB200_GEN_PER_LAYER_KERNELS |
+                                 SNB200_GEN_SEPARATE_HEAD | SNB200_GEN_WORKSPACE_PRIMED;
+
 }  // namespace snb
 
 using namespace snb;
@@ -245,6 +250,7 @@ SNB_API int snb200_generator_forward(int b, int n, int layout, const float *x, i
                                      const snb200_layer *fc, int training, float *out, int out_transpose_inner, float *feat, int flags,
                                      void *workspace, size_t workspace_bytes, snb200_stream_t stream)
 {
+    SNB_REQUIRE((flags & ~kGenFlagsDefined) == 0, "generator_forward: flags 0x%x set bits outside the defined set 0x%x", flags, kGenFlagsDefined);
     int rc = check_layers("generator_forward", num_conv, conv, SNB200_MAX_CONV_LAYERS);
     if (rc) return rc;
     rc = check_layers("generator_forward", num_fc, fc, SNB200_MAX_FC_LAYERS);
@@ -282,6 +288,7 @@ SNB_API int snb200_generator_train_forward(int b, int n, int layout, const float
                                            const snb200_layer *fc, float *out, int out_transpose_inner, float *feat, float *const *zsave, int flags,
                                            void *workspace, size_t workspace_bytes, snb200_stream_t stream)
 {
+    SNB_REQUIRE((flags & ~kGenFlagsDefined) == 0, "generator_train_forward: flags 0x%x set bits outside the defined set 0x%x", flags, kGenFlagsDefined);
     SNB_REQUIRE(zsave != nullptr, "generator_train_forward: zsave is null");
     int rc = check_layers("generator_train_forward", num_conv, conv, SNB200_MAX_CONV_LAYERS);
     if (rc) return rc;

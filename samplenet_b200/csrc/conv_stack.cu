@@ -29,6 +29,7 @@
 //     keeps them in registers.
 // Applicable to widths <= 128 with K in {32, 64, 128} and up to 16 slices per CTA; otherwise the per-layer kernels are used.
 #include "encoder_internal.cuh"
+#include "tcgen05.cuh"
 #include <cooperative_groups.h>
 #include <string.h>
 #include <stdlib.h>
@@ -90,40 +91,6 @@ struct CsParams {
     int head_rows;                      // batch rows the FC head stages per pass (32 ... 128, a multiple of 32)
     int dbg;                            // bring-up switches (env SNB200_CS_DEBUG; 0 in the product): 1 = skip the statistics atomics (timing experiments only)
 };
-
-// ---- tcgen05 helpers (same encodings as encoder_tc.cu, validated against fp64 in tests/test_gpu_parity.py::test_tc_gemm_3xtf32)
-__device__ __forceinline__ void cs_tmem_alloc(uint32_t *smem_dst, uint32_t ncols)
-{
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(smem_dst)), "r"(ncols) : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-}
-__device__ __forceinline__ void cs_tmem_dealloc(uint32_t taddr, uint32_t ncols)
-{
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(taddr), "r"(ncols) : "memory");
-}
-__device__ __forceinline__ void cs_fence_before() { asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory"); }
-__device__ __forceinline__ void cs_fence_after() { asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory"); }
-__device__ __forceinline__ void cs_commit(uint64_t *bar)
-{
-    asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(smem_u32(bar)) : "memory");
-}
-__device__ __forceinline__ void cs_ld8_issue(uint32_t taddr, uint32_t *r)
-{
-    asm volatile("tcgen05.ld.sync.aligned.32x32b.x8.b32 {%0, %1, %2, %3, %4, %5, %6, %7}, [%8];"
-                 : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7])
-                 : "r"(taddr)
-                 : "memory");
-}
-__device__ __forceinline__ void cs_ld_wait() { asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory"); }
-__host__ __device__ constexpr uint32_t cs_idesc(int M, int N)
-{
-    return (1u << 4) | (2u << 7) | (2u << 10) | ((uint32_t)(N >> 3) << 17) | ((uint32_t)(M >> 4) << 24);
-}
-constexpr unsigned kCsDescHi = (64u) | (1u << 14) | (2u << 29);
-__device__ __forceinline__ uint64_t cs_sdesc(uint32_t smem_addr)
-{
-    return (uint64_t)((smem_addr >> 4) & 0x3fffu) | (1ull << 16) | ((uint64_t)kCsDescHi << 32);
-}
 
 // bounded waits: a protocol bug must not hang the GPU box -- trap instead (surfaces as a launch failure in the next API call)
 __device__ __forceinline__ void cs_mbar_wait(uint64_t *bar, uint32_t parity)
@@ -311,26 +278,6 @@ __device__ __forceinline__ void cs_fx_collect(double *stats, int C, int ch, unsi
     sumsq = (double)(long long)(b & kFxFieldMask) * (1.0 / 512.0) + (double)(long long)(c & kFxFieldMask) * (1.0 / 281474976710656.0);
 }
 
-// A-from-TMEM form: D[tmem] (+)= A[tmem, 128 lanes x 8 columns] . B[smem descriptor]
-__device__ __forceinline__ void cs_umma_ts(uint32_t tmem_d, uint32_t tmem_a, uint64_t bdesc, uint32_t idesc, uint32_t accumulate)
-{
-    asm volatile(
-        "{\n"
-        ".reg .pred p;\n"
-        "setp.ne.b32 p, %4, 0;\n"
-        "tcgen05.mma.cta_group::1.kind::tf32 [%0], [%1], %2, %3, p;\n"
-        "}\n" ::"r"(tmem_d),
-        "r"(tmem_a), "l"(bdesc), "r"(idesc), "r"(accumulate)
-        : "memory");
-}
-__device__ __forceinline__ void cs_st8(uint32_t taddr, const uint32_t *r)
-{
-    asm volatile("tcgen05.st.sync.aligned.32x32b.x8.b32 [%0], {%1, %2, %3, %4, %5, %6, %7, %8};" ::"r"(taddr), "r"(r[0]), "r"(r[1]), "r"(r[2]),
-                 "r"(r[3]), "r"(r[4]), "r"(r[5]), "r"(r[6]), "r"(r[7])
-                 : "memory");
-}
-__device__ __forceinline__ void cs_st_wait() { asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory"); }
-
 __device__ long long g_cs_ts[64];
 #define CS_TS(i) do { if (blockIdx.x == 0 && threadIdx.x == 0 && (i) < 64) g_cs_ts[(i)] = clock64(); } while (0)
 
@@ -368,11 +315,11 @@ __device__ __forceinline__ void cs_store_w(uint32_t tmem_lane_base, int g, int K
                 hi[i] = __float_as_uint(h);
                 lo[i] = __float_as_uint(v - h);
             }
-            cs_st8(tmem_lane_base + kCsColWhi + (uint32_t)(g * K4 + i8 * 8), hi);
-            cs_st8(tmem_lane_base + kCsColWlo + (uint32_t)(g * K4 + i8 * 8), lo);
+            tmem_st8(tmem_lane_base + kCsColWhi + (uint32_t)(g * K4 + i8 * 8), hi);
+            tmem_st8(tmem_lane_base + kCsColWlo + (uint32_t)(g * K4 + i8 * 8), lo);
         }
     }
-    cs_st_wait();
+    tmem_st_wait();
 }
 
 // (B) of the layer loop: this thread's channel = column k of the B operand: normalise, split and store its npt points into a ring slot.
@@ -440,21 +387,21 @@ __device__ __forceinline__ void cs_issue_chunk(unsigned char *smem_raw, uint32_t
 {
     const uint32_t gi = gchunk + (uint32_t)c, slot = gi % kCsRing, use = gi / kCsRing;
     cs_mbar_wait(&bar_full[slot], use & 1u);
-    cs_fence_after();
+    tc_fence_after();
     if (lane == 0) {
         const uint32_t sb = smem_u32(smem_raw) + slot * slot_bytes;
-        const uint64_t b_hi = cs_sdesc(sb), b_lo = cs_sdesc(sb + (uint32_t)kCsLoPlane);
+        const uint64_t b_hi = make_sdesc(sb, kDescHiSw128), b_lo = make_sdesc(sb + (uint32_t)kCsLoPlane, kDescHiSw128);
         const uint32_t a_hi = tmem0 + kCsColWhi + (uint32_t)(c * 32), a_lo = tmem0 + kCsColWlo + (uint32_t)(c * 32);
 #pragma unroll
         for (int ks = 0; ks < 4; ks++) {   // K = 8 tf32 per step: +8 TMEM columns (A), +32 bytes = +2 in the 16-byte address field (B)
             const uint64_t o = (uint64_t)(ks * 2);
             const uint32_t ka = (uint32_t)(ks * 8);
-            cs_umma_ts(tmem0, a_lo + ka, b_hi + o, idesc, (c > 0 || ks > 0) ? 1u : 0u);
-            cs_umma_ts(tmem0, a_hi + ka, b_lo + o, idesc, 1u);
-            cs_umma_ts(tmem0, a_hi + ka, b_hi + o, idesc, 1u);
+            umma_tf32_ts(tmem0, a_lo + ka, b_hi + o, idesc, (c > 0 || ks > 0) ? 1u : 0u);
+            umma_tf32_ts(tmem0, a_hi + ka, b_lo + o, idesc, 1u);
+            umma_tf32_ts(tmem0, a_hi + ka, b_hi + o, idesc, 1u);
         }
-        cs_commit(&bar_ring[slot]);
-        if (c == nchunks - 1) cs_commit(bar_acc);
+        umma_commit(&bar_ring[slot]);
+        if (c == nchunks - 1) umma_commit(bar_acc);
     }
     __syncwarp();
 }
@@ -497,7 +444,7 @@ __global__ void __launch_bounds__(kCsThreadsAll, 1) conv_stack_kernel(const __gr
     const uint32_t slot_bytes = kCsSlotBytes;
 
     CS_TS(0);
-    if (warp == 0) cs_tmem_alloc(&tmem_base_smem, 512);
+    if (warp == 0) tmem_alloc(&tmem_base_smem, 512);
     if (tid == 0) {
         for (int s = 0; s < kCsRing; s++) { mbar_init(&bar_full[s], 128); mbar_init(&bar_ring[s], 1); }
         mbar_init(&bar_acc, 1);
@@ -533,9 +480,9 @@ __global__ void __launch_bounds__(kCsThreadsAll, 1) conv_stack_kernel(const __gr
         for (int e = tid; e < L1.c_out * 3; e += kCsProducers) sW1[e] = __ldg(L1.weight + e);
         for (int e = tid; e < L1.c_out; e += kCsProducers) sB1[e] = L1.bias ? __ldg(L1.bias + e) : 0.f;
     }
-    cs_fence_before();
+    tc_fence_before();
     __syncthreads();
-    cs_fence_after();
+    tc_fence_after();
     const uint32_t tmem0 = tmem_base_smem;
     const uint32_t tmem_lane = tmem0 + ((uint32_t)(q * 32) << 16);
     unsigned barrier_epoch = 0;
@@ -593,7 +540,7 @@ __global__ void __launch_bounds__(kCsThreadsAll, 1) conv_stack_kernel(const __gr
     }
     if (producer) {   // weights of the first tensor layer into tensor memory
         cs_store_w(tmem_lane, g, P.L[1].c_in >> 2, wreg);
-        cs_fence_before();
+        tc_fence_before();
         cs_mbar_arrive(&bar_w);
     }
     if (need_stats && L1.has_bn) {
@@ -691,10 +638,10 @@ __global__ void __launch_bounds__(kCsThreadsAll, 1) conv_stack_kernel(const __gr
             }
             CS_TS(3 + (l - 1) * 8 + 1);
             // (B) MMA issue (warp kCsIssuerWarp, chunks in order) around the operand preparation (every warp that owns a K chunk)
-            const uint32_t idesc = cs_idesc(128, ppc);
+            const uint32_t idesc = make_idesc_tf32(128, ppc);
             if (issuer) {
                 cs_mbar_wait(&bar_w, (uint32_t)(l - 1) & 1u);   // every thread's slice of this layer's weights is in tensor memory
-                cs_fence_after();
+                tc_fence_after();
             }
             const float bias = (ch < N && Lc.bias) ? __ldg(Lc.bias + ch) : 0.f;
             float sumL = 0.f, sqL = 0.f;                                     // (kMulti) this thread's statistics over all of its slices
@@ -754,7 +701,7 @@ __global__ void __launch_bounds__(kCsThreadsAll, 1) conv_stack_kernel(const __gr
                     const uint32_t gi = gchunk + (uint32_t)q, slot = gi % kCsRing, use = gi / kCsRing;
                     if (use > 0) {   // the MMAs that read this ring slot last time must have completed
                         cs_mbar_wait(&bar_ring[slot], (use - 1) & 1u);
-                        cs_fence_after();
+                        tc_fence_after();
                     }
                     uint32_t adr[8];
                     const uint32_t sbase = smem_u32(smem_raw) + slot * slot_bytes;
@@ -762,7 +709,7 @@ __global__ void __launch_bounds__(kCsThreadsAll, 1) conv_stack_kernel(const __gr
                     for (int i = 0; i < 8; i++) adr[i] = sbase + toff[i];
                     if (!last) CS_TS(3 + (l - 1) * 8 + 7);
                     cs_write_chunk(v, sc, sh, Lp.relu ? 0.f : -INFINITY, npt, adr);
-                    cs_fence_before();     // this thread's tcgen05.ld of the previous accumulator are complete (wait::ld) and ordered
+                    tc_fence_before();     // this thread's tcgen05.ld of the previous accumulator are complete (wait::ld) and ordered
                     fence_proxy_async();   // generic-proxy writes -> visible to the tensor core
                     cs_mbar_arrive(&bar_full[slot]);
                 }
@@ -774,12 +721,12 @@ __global__ void __launch_bounds__(kCsThreadsAll, 1) conv_stack_kernel(const __gr
                 // (D) every MMA of this slice has completed
                 cs_mbar_wait(&bar_acc, acc_uses & 1u);
                 acc_uses++;
-                cs_fence_after();
+                tc_fence_after();
                 CS_TS(3 + (l - 1) * 8 + 3);
                 // (E) the next layer's weights replace this layer's in tensor memory
                 if (!last && lastslice) {
                     cs_store_w(tmem_lane, g, P.L[l + 1].c_in >> 2, wreg);
-                    cs_fence_before();
+                    tc_fence_before();
                     cs_mbar_arrive(&bar_w);
                 }
                 // (F) the accumulator: lane = channel, this thread's npt columns -> registers (+bias); statistics / extrema on the way
@@ -788,9 +735,9 @@ __global__ void __launch_bounds__(kCsThreadsAll, 1) conv_stack_kernel(const __gr
                 if (q * 32 < N) {
 #pragma unroll
                     for (int jb = 0; jb < kCsNPT / 8; jb++)
-                        if (jb * 8 < npt) cs_ld8_issue(tmem_lane + (uint32_t)(col0 + jb * 8), v + jb * 8);
-                    cs_ld_wait();
-                    cs_fence_before();   // the next MMA into this accumulator overwrites these columns: ordered through a CTA barrier below
+                        if (jb * 8 < npt) tmem_ld8(tmem_lane + (uint32_t)(col0 + jb * 8), v + jb * 8);
+                    tmem_ld_wait();
+                    tc_fence_before();   // the next MMA into this accumulator overwrites these columns: ordered through a CTA barrier below
                     float sum = 0.f, sq = 0.f;
                     if (nvalid == npt) {   // (every slice but the last: all columns are real points)
 #pragma unroll
@@ -893,7 +840,7 @@ __global__ void __launch_bounds__(kCsThreadsAll, 1) conv_stack_kernel(const __gr
     }
 
     // every commit has been observed through bar_acc; tensor memory is released at the end of the kernel (off the head's critical path)
-    cs_fence_before();
+    tc_fence_before();
     __syncthreads();
     CS_TS(35);
 
@@ -909,7 +856,7 @@ __global__ void __launch_bounds__(kCsThreadsAll, 1) conv_stack_kernel(const __gr
     if (!P.fuse_head) {   // stand-alone conv stack: the consumers (cluster head kernel, backward pass) read the canonical statistics block
         const CsLayer &LL = P.L[P.num_layers - 1];
         if (blockIdx.x == 0 && need_stats && LL.has_bn && tid < 2 * LL.c_out) LL.stats[tid] = cs_stat(LL.stats, 2 * LL.c_out, tid, 1);
-        if (warp == 0) cs_tmem_dealloc(tmem0, 512);
+        if (warp == 0) tmem_dealloc(tmem0, 512);
         return;
     }
     const HeadParams &H = P.H;
@@ -1242,7 +1189,7 @@ __global__ void __launch_bounds__(kCsThreadsAll, 1) conv_stack_kernel(const __gr
             base = (base + H.ru_c[l]) % gn;
         }
     }
-    if (warp == 0) cs_tmem_dealloc(tmem0, 512);
+    if (warp == 0) tmem_dealloc(tmem0, 512);
     if (P.self_clean) {   // the last CTA to leave puts the moments, the barrier word and the exit word back to zero for the next launch
         __syncthreads();
         if (tid == 0) {

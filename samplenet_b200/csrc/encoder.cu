@@ -41,26 +41,6 @@ struct ConvLayerParams {
     float *tile_max, *tile_min;    // (b*tiles_per_cloud, c_out) or nullptr
 };
 
-// scale/shift of a BatchNorm given either batch statistics or running statistics
-__device__ __forceinline__ void bn_scale_shift(const double *stats, int c_total, int c, double count, const float *gamma, const float *beta,
-                                               const float *run_mean, const float *run_var, float eps, int training, float &scale, float &shift)
-{
-    float mean, var;
-    if (training) {
-        const double m = stats[c] / count;
-        double v = stats[c_total + c] / count - m * m;
-        if (v < 0) v = 0;
-        mean = (float)m;
-        var = (float)v;
-    } else {
-        mean = run_mean[c];
-        var = run_var[c];
-    }
-    const float invstd = 1.0f / sqrtf(var + eps);
-    scale = gamma[c] * invstd;
-    shift = beta[c] - mean * scale;
-}
-
 // CC = output channels per CTA (64 or 128); thread tile 8 points x 8 channels; TP = points per CTA.
 template <int CC>
 __global__ void __launch_bounds__(kEncThreads) conv_layer_kernel(const __grid_constant__ ConvLayerParams P)

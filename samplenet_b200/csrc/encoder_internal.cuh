@@ -1,4 +1,4 @@
-// encoder_internal.cuh -- declarations shared by encoder.cu (CUDA-core path), encoder_tc.cu (tcgen05 path) and generator.cu.
+// encoder_internal.cuh -- declarations shared by encoder.cu (CUDA-core path), encoder_tc.cu (tcgen05 path), conv_stack.cu and generator.cu.
 #pragma once
 #include "common.cuh"
 
@@ -87,11 +87,26 @@ int launch_conv_stack(int b, int n, int layout, const float *x, int nconv, const
                       double *mom, unsigned *barrier, float *tile_max, float *tile_min, int *tiles_per_cloud_out, const HeadParams *head,
                       char *clean_ptr, size_t clean_bytes, cudaStream_t stream, float *const *zsave = nullptr, float *const *act = nullptr);
 
-namespace v1 {   // round-1 conv-stack kernel (conv_stack_v1.cu), selected by SNB200_GEN_CONV_STACK_V1
-bool conv_stack_supported(int b, int n, int nconv, const snb200_layer *conv);
-int launch_conv_stack(int b, int n, int layout, const float *x, int nconv, const snb200_layer *conv, int training, double *const *stats,
-                      double *mom, unsigned *barrier, float *tile_max, float *tile_min, int *tiles_per_cloud_out, const HeadParams *head,
-                      char *clean_ptr, size_t clean_bytes, cudaStream_t stream);
-}  // namespace v1
+#ifdef __CUDACC__
+// scale/shift of a BatchNorm given either batch statistics or running statistics
+__device__ __forceinline__ void bn_scale_shift(const double *stats, int c_total, int c, double count, const float *gamma, const float *beta,
+                                               const float *run_mean, const float *run_var, float eps, int training, float &scale, float &shift)
+{
+    float mean, var;
+    if (training) {
+        const double m = stats[c] / count;
+        double v = stats[c_total + c] / count - m * m;
+        if (v < 0) v = 0;
+        mean = (float)m;
+        var = (float)v;
+    } else {
+        mean = run_mean[c];
+        var = run_var[c];
+    }
+    const float invstd = 1.0f / sqrtf(var + eps);
+    scale = gamma[c] * invstd;
+    shift = beta[c] - mean * scale;
+}
+#endif  // __CUDACC__
 
 }  // namespace snb

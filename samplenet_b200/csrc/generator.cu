@@ -27,23 +27,6 @@ constexpr int kHeadThreads = 256;      // 8 warps = 8 K slices; lanes = 8 row qu
 constexpr int kHeadChPerCta = 16;
 constexpr int kHeadMaxCluster = 16;
 
-__device__ __forceinline__ void head_bn_scale_shift(const double *stats, int c_total, int c, double count, const float *gamma, const float *beta,
-                                                    const float *run_mean, const float *run_var, float eps, int training, float &scale, float &shift)
-{
-    float mean, var;
-    if (training) {
-        const double m = stats[c] / count;
-        double v = stats[c_total + c] / count - m * m;
-        if (v < 0) v = 0;
-        mean = (float)m; var = (float)v;
-    } else {
-        mean = run_mean[c]; var = run_var[c];
-    }
-    const float invstd = 1.0f / sqrtf(var + eps);
-    scale = gamma[c] * invstd;
-    shift = beta[c] - mean * scale;
-}
-
 // bring-up instrumentation: SM-clock timestamps of CTA 0 / thread 0 at phase boundaries (read with snb200_debug_head_timestamps)
 __device__ long long g_head_ts[64];
 #define HEAD_TS(i) do { if (blockIdx.x == 0 && threadIdx.x == 0 && (i) < 64) g_head_ts[(i)] = clock64(); } while (0)
@@ -477,8 +460,7 @@ int launch_generator_forward(int b, int n, int layout, const float *x, int nconv
                              float *const *zsave)
 {
     GenWorkspace W = carve_gen_ws(workspace, b, n, nconv, conv, nfc, fc);
-    const bool use_v1 = (flags & SNB200_GEN_CONV_STACK_V1) != 0 && zsave == nullptr;
-    const bool cs_ok = use_v1 ? v1::conv_stack_supported(b, n, nconv, conv) : conv_stack_supported(b, n, nconv, conv);
+    const bool cs_ok = conv_stack_supported(b, n, nconv, conv);
     const bool coop = !(flags & (SNB200_GEN_EXACT_FP32 | SNB200_GEN_PER_LAYER_KERNELS | SNB200_GEN_PROFILE_SKIP_CONV)) && tc_stack_supported(nconv, conv) && cs_ok;
     // SNB200_GEN_WORKSPACE_PRIMED: the caller keeps this workspace for this call sequence and its first 256 bytes (moments, barrier
     // and exit words) are zero -- freshly zeroed, or as the previous PRIMED call left them.  The persistent kernel then cleans the
@@ -495,17 +477,15 @@ int launch_generator_forward(int b, int n, int layout, const float *x, int nconv
     const bool use_tc = !(flags & SNB200_GEN_EXACT_FP32) && tc_stack_supported(nconv, conv);
     int tpc = 0;
     if (flags & SNB200_GEN_PROFILE_SKIP_CONV) {
-        tpc = (use_tc && cs_ok) ? (use_v1 ? (n + 127) / 128 : conv_stack_slots_per_cloud(b, n)) : use_tc ? tc_tiles_per_cloud(n) : (n + (conv[nconv - 1].c_out > 64 ? 128 : 256) - 1) / (conv[nconv - 1].c_out > 64 ? 128 : 256);
+        tpc = (use_tc && cs_ok) ? conv_stack_slots_per_cloud(b, n) : use_tc ? tc_tiles_per_cloud(n) : (n + (conv[nconv - 1].c_out > 64 ? 128 : 256) - 1) / (conv[nconv - 1].c_out > 64 ? 128 : 256);
     } else if (use_tc && !(flags & SNB200_GEN_PER_LAYER_KERNELS) && cs_ok) {
         // one persistent cooperative launch for the conv stack AND (unless profiling flags split them) the pool + FC head
         HeadParams H;
         bool fuse_head = !(flags & (SNB200_GEN_PROFILE_SKIP_HEAD | SNB200_GEN_SEPARATE_HEAD)) && b <= 256;
         for (int l = 0; l < nfc; l++) fuse_head = fuse_head && fc[l].c_in <= 1024;
-        if (fuse_head) fill_head_params(H, b, n, use_v1 ? (n + 127) / 128 : conv_stack_slots_per_cloud(b, n), nconv, conv, nfc, fc, training, out, out_transpose_inner, feat_out, W);
-        int rc = use_v1 ? v1::launch_conv_stack(b, n, layout, x, nconv, conv, training, W.stats, W.mom, W.counter, W.tile_max, W.tile_min, &tpc,
-                                                fuse_head ? &H : nullptr, (self_clean && fuse_head) ? W.stats_base + 256 : nullptr, W.stats_bytes - 256, stream)
-                        : launch_conv_stack(b, n, layout, x, nconv, conv, training, W.stats, W.mom, W.counter, W.tile_max, W.tile_min, &tpc,
-                                            fuse_head ? &H : nullptr, (self_clean && fuse_head) ? W.stats_base + 256 : nullptr, W.stats_bytes - 256, stream, zsave, W.act);
+        if (fuse_head) fill_head_params(H, b, n, conv_stack_slots_per_cloud(b, n), nconv, conv, nfc, fc, training, out, out_transpose_inner, feat_out, W);
+        int rc = launch_conv_stack(b, n, layout, x, nconv, conv, training, W.stats, W.mom, W.counter, W.tile_max, W.tile_min, &tpc,
+                                   fuse_head ? &H : nullptr, (self_clean && fuse_head) ? W.stats_base + 256 : nullptr, W.stats_bytes - 256, stream, zsave, W.act);
         if (rc) return rc;
         if (fuse_head) return SNB200_OK;
     } else if (use_tc) {

@@ -539,12 +539,7 @@ class primed_workspaces:
         return False
 
 
-# Which persistent conv-stack kernel the default generator path uses: 2 = transposed GEMMs (round 2), 1 = the round-1 kernel.
-CONV_STACK_VERSION = 1 if os.environ.get("SNB200_CONV_STACK", "") == "v1" else 2
-
-
-def generator_forward(x, layout, conv_specs, fc_specs, training, out_transpose_inner=0, exact_fp32=False, _profile_flags=0, per_layer_kernels=False, separate_head=False,
-                      conv_stack_version=None):
+def generator_forward(x, layout, conv_specs, fc_specs, training, out_transpose_inner=0, exact_fp32=False, _profile_flags=0, per_layer_kernels=False, separate_head=False):
     """x (B,N,3)/(B,3,N) -> (out (B, c_out_last), feat (B, c_conv_last)): conv stack + max-pool + FC head in ONE C-ABI call.
     Default: conv layers on the tensor cores (tcgen05, 3xTF32) + cluster-fused FC head; exact_fp32=True: CUDA-core conv stack."""
     lay = _layout(layout)
@@ -569,8 +564,7 @@ def generator_forward(x, layout, conv_specs, fc_specs, training, out_transpose_i
         feat = torch.empty(b, conv[len(conv_specs) - 1].c_out, device=dev)
         out = torch.empty(b, fc[len(fc_specs) - 1].c_out, device=dev)
         check(lib().snb200_generator_forward(b, n, lay, _p(x), len(conv_specs), conv, len(fc_specs), fc, int(bool(training)), _p(out),
-                                             int(out_transpose_inner), _p(feat), (_lib.GEN_EXACT_FP32 if exact_fp32 else 0) | (8 if per_layer_kernels else 0) | (16 if separate_head else 0) | int(_profile_flags) | primed |
-                                             (64 if (conv_stack_version or CONV_STACK_VERSION) == 1 else 0), _p(ws), wsb,
+                                             int(out_transpose_inner), _p(feat), (_lib.GEN_EXACT_FP32 if exact_fp32 else 0) | (8 if per_layer_kernels else 0) | (16 if separate_head else 0) | int(_profile_flags) | primed, _p(ws), wsb,
                                              _stream()), "generator_forward")
     del keep1, keep2
     return out, feat

@@ -73,6 +73,18 @@ def test_primed_workspace_context_is_scoped_and_nestable(sb):
     assert re.search(r"#define\s+SNB200_GEN_WORKSPACE_PRIMED\s+32", hdr)
 
 
+def test_generator_rejects_undefined_flag_bits(sb):
+    """A generator flag bit the header does not define is an error, checked before any other argument (no launch), so a caller that
+    still sets the retired bit 64 is told so instead of silently getting a different kernel."""
+    lib = sb._lib.lib()
+    rc = lib.snb200_generator_forward(2, 16, 0, None, 5, None, 4, None, 1, None, 0, None, 64, None, 0, None)
+    assert rc == -1
+    assert "flags" in lib.snb200_last_error().decode()
+    rc = lib.snb200_generator_train_forward(2, 16, 0, None, 5, None, 4, None, None, 0, None, None, 64, None, 0, None)
+    assert rc == -1
+    assert "flags" in lib.snb200_last_error().decode()
+
+
 def test_samplenet_constructor_contract(sb):
     with pytest.raises(ValueError):
         sb.SampleNet(64, 128, 8, input_shape="nbc")

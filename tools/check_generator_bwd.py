@@ -4,7 +4,6 @@ import os, sys, time
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import torch
 import samplenet_b200 as sb
-sb.ops.CONV_STACK_VERSION = 2
 
 torch.manual_seed(0)
 ok = True

@@ -4,7 +4,6 @@ import os, sys
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import torch
 import samplenet_b200 as sb
-sb.ops.CONV_STACK_VERSION = 2
 torch.manual_seed(0)
 for (b, n, m, layout) in [(64, 512, 64, "bnc"), (48, 512, 64, "bnc"), (64, 256, 64, "bnc")]:
     net = sb.SampleNet(m, 128, group_size=8, input_shape=layout, output_shape=layout).cuda().train()

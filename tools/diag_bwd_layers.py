@@ -4,7 +4,6 @@ import os, sys
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import numpy as np, torch
 import samplenet_b200 as sb
-sb.ops.CONV_STACK_VERSION = 2
 b, n, m, layout = [int(v) if v.isdigit() else v for v in (sys.argv[1:5] if len(sys.argv) >= 5 else ["64", "512", "64", "bnc"])]
 torch.manual_seed(b + n)
 net = sb.SampleNet(m, 128, group_size=8, input_shape=layout, output_shape=layout).cuda().train()

@@ -3,7 +3,7 @@
 N=${1:-2}
 TAG=${2:-r2}
 mkdir -p gpurun_out
-export SNB200_CONV_STACK=${SNB200_CONV_STACK:-v2} SNB200_GENERATOR_BACKWARD=${SNB200_GENERATOR_BACKWARD:-cuda}
+export SNB200_GENERATOR_BACKWARD=${SNB200_GENERATOR_BACKWARD:-cuda}
 timeout -k 10 600 python -m torch.distributed.run --nnodes=1 --nproc-per-node $N --master-addr 127.0.0.1 --master-port 29533 tools/bench_configs.py --only train \
   > gpurun_out/${TAG}_train_n${N}.jsonl 2> gpurun_out/${TAG}_train_n${N}.err; echo "train n=$N rc=$?"
 cat gpurun_out/${TAG}_train_n${N}.jsonl; tail -5 gpurun_out/${TAG}_train_n${N}.err
